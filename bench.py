@@ -6,7 +6,7 @@ Workload = BASELINE.json configs[1]: one environment per GPU, 640x480 RGB-D, 100
 architecture: no checkpoint exists offline), weighted-average fusion
 (use_max_confidence=False, the policies' setting).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--batch B]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--batch B] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU, env shards, NO step-path collective;
 NCCL only for the barrier and the max-over-ranks of the timing).  Prints ONE JSON line.
@@ -196,6 +196,7 @@ def run_b200(args):
         j = i % NFRAMES
         cos = itm.cosine_device(rgb[j], PROMPT)
         eng.update(cos.double().view(B, 1), depth[j], tfs[j], MIN_D, MAX_D, FOV)
+        return cos
 
     def barrier():
         if world > 1:
@@ -217,10 +218,12 @@ def run_b200(args):
     barrier()
     e0.record()
     for i in range(K):
-        step_device(Wm + i)
+        cos = step_device(Wm + i)
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:         # before the legs below reuse the engines' buffers
+        dump_outputs(args.dump_outputs, cos, eng)
     from vlfm_b200.utils.dist import aggregate_throughput, gather_metrics, max_over_ranks
 
     ms_local = ms
@@ -334,6 +337,22 @@ def run_b200(args):
     emit(extra)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, cos, eng):
+    """What the timed path handed its caller after the last timed step, as .npy files: the ITC cosine of every environment
+    (cosine.npy, [B]) and the confidence / value grids (confidence.npy [n,G,G], value.npy [n,G,G,1], float32 as kept in HBM) of
+    the first n environments, n as large as keeps the files under 64 MB (all of them up to 7 envs at G=1000)."""
+    os.makedirs(out_dir, exist_ok=True)
+    cosine = cos.float().cpu().numpy()
+    per_env = (eng.conf[0].numel() + eng.value[0].numel()) * 4
+    n = max(1, min(eng.batch, (DUMP_BYTES - cosine.nbytes - 4096) // per_env))
+    np.save(os.path.join(out_dir, "cosine.npy"), cosine)
+    np.save(os.path.join(out_dir, "confidence.npy"), eng.conf[:n].cpu().numpy())
+    np.save(os.path.join(out_dir, "value.npy"), eng.value[:n].cpu().numpy())
 
 
 EXTRAS_MARK = "VLFM_EXTRAS_JSON "
@@ -579,7 +598,14 @@ def main():
     ap.add_argument("--extra-batch", type=int, default=32, help="envs per GPU of the extra slices")
     ap.add_argument("--extra-multi", action="store_true", help="run the extra workloads on every rank of a multi-GPU launch too")
     ap.add_argument("--extras-child", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the cosines and value-map grids of the last timed step as DIR/<name>.npy (rank 0's environments); "
+                         "the inputs are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the b200 path")
     if args.extras_child:
         extras_child(args)
     elif args.impl == "reference":

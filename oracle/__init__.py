@@ -18,8 +18,10 @@ Contents
                         fog-of-war / frontier half is UNPINNED, see DESIGN.md).
 ``blip2_oracle``        architecture-equivalent fp32 BLIP-2 ITC forward built on
                         HF transformers (LAVIS is absent: parity UNPINNED w.r.t. LAVIS).
-``ref_import``          imports the real reference from /root/reference (container only;
-                        used to pin the restatements and to generate tests/golden/*).
+``ref_import``          imports the real reference from a checkout named by VLFM_REFERENCE
+                        (used only by ``make_golden`` to generate tests/golden/*).
+``golden``              compact storage of, and exact comparison with, the stored
+                        reference outputs under tests/golden/.
 
 Pinning status is recorded per module in its header and in DESIGN.md.
 """

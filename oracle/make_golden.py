@@ -1,9 +1,11 @@
-"""Generate tests/golden/*.npz by running the REAL reference (build container only).
+"""Generate tests/golden/*.npz by running the REAL reference.
 
-Usage:  PYTHONPATH=/root/repo python oracle/make_golden.py
-Needs /root/reference.  Inputs are regenerated from vlfm_b200.utils.synthetic with the
-recorded seeds (an input checksum is stored so generator drift is detected); outputs
-are stored sparsely (flat indices + values of non-zero cells).
+Usage:  VLFM_REFERENCE=<checkout of the original vlfm repository> python oracle/make_golden.py
+Inputs are regenerated from vlfm_b200.utils.synthetic with the recorded seeds (an input
+checksum is stored so generator drift is detected); outputs are stored sparsely (flat
+indices + values of non-zero cells, bit-packed 0/1 grids).  The ref_*.npz case sets are
+produced by the tests' own run_* functions (tests/test_*.py), called here with the
+reference classes and there with the oracle / product classes.
 """
 from __future__ import annotations
 
@@ -13,12 +15,13 @@ import sys
 
 import numpy as np
 
-sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 
-from oracle import ref_import  # noqa: E402
+from oracle import golden, ref_import  # noqa: E402
 from vlfm_b200.utils.synthetic import focal_from_hfov, trajectory  # noqa: E402
 
-OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+OUT = os.path.join(ROOT, "tests", "golden")
 FOV = float(np.deg2rad(79.0))
 
 VALUE_CASES = [
@@ -71,16 +74,67 @@ def value_cases() -> None:
         print(name, "conf nz", ci.size, "value nz", vi.size)
 
 
-def obstacle_cases() -> None:
-    try:
-        from oracle.make_golden_obstacle import obstacle_cases as run
-    except ImportError:
-        return
-    run(OUT)
+def _save(name: str, arrays) -> None:
+    path = os.path.join(OUT, name + ".npz")
+    golden.save(path, arrays)
+    print(name, len(arrays), "arrays", os.path.getsize(path), "bytes")
+
+
+def live_cases() -> None:
+    """The reference side of the tests that compare a restatement with the reference class on the same inputs."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import test_base_map
+    import test_frontier_map
+    import test_oracle_explore
+    import test_oracle_object_map
+    import test_oracle_obstacle
+    import test_oracle_value_map
+
+    RV = ref_import.value_map_class()
+
+    def value_map(ch, size, maxc, fus, ppm=None):
+        RV._confidence_masks.clear()
+        m = RV(ch, size=size, use_max_confidence=maxc, fusion_type=fus)
+        if ppm is not None:            # value_map.py:65 fixes 20 px/m; the cone cache (value_map.py:339) is per class
+            m.pixels_per_meter = ppm
+        return m
+
+    _save("ref_value_map_live", test_oracle_value_map.run_live_cases(value_map))
+    _save("ref_value_map_ppm40", test_oracle_value_map.run_ppm40(lambda size: value_map(1, size, False, "default", ppm=40)))
+    RV._confidence_masks.clear()
+
+    RO = ref_import.obstacle_map_class()
+    out = {}
+    for hole in (-1, 100000):
+        out.update({f"hole{hole}_{k}": v for k, v in test_oracle_obstacle.run_obstacle_half(RO, hole).items()})
+    _save("ref_obstacle_half", out)
+    _save("ref_explore", test_oracle_explore.run_reference_class_case(RO))
+
+    RF = ref_import.frontier_map_class(test_frontier_map.ScriptedEncoder)
+    out = {}
+    for seed in (0, 1, 2):
+        fm = RF()
+        fm.frontiers = []              # a class attribute in the reference
+        out.update({f"s{seed}_{k}": v for k, v in test_frontier_map.run_stream(fm, seed).items()})
+    _save("ref_frontier_map", out)
+
+    R = ref_import.object_map_module().ObjectPointCloudMap
+
+    def object_map():
+        m = R(erosion_size=2)
+        m.reset()
+        return m
+
+    out = {}
+    for use_dbscan in (True, False):
+        out.update({f"dbscan{int(use_dbscan)}_{k}": v for k, v in test_oracle_object_map.run_scenarios(object_map, use_dbscan).items()})
+    _save("ref_object_map", out)
+
+    _save("ref_base_map", test_base_map.run_conversions(ref_import.base_map_class()(size=1000)))
 
 
 if __name__ == "__main__":
-    assert ref_import.available(), "needs /root/reference"
+    assert ref_import.available(), "set VLFM_REFERENCE to a checkout of the original vlfm repository"
     os.makedirs(OUT, exist_ok=True)
     value_cases()
-    obstacle_cases()
+    live_cases()

@@ -2,8 +2,8 @@
 
 TEST INFRASTRUCTURE (see oracle/__init__.py).
 
-Pinning: everything except the DBSCAN call is checked bit-for-bit against the REAL reference class imported from
-/root/reference with a stub ``open3d`` module injected (tests/test_oracle_object_map.py).  ``open3d`` itself (``open3d``,
+Pinning: everything except the DBSCAN call is checked bit-for-bit against what the REAL reference class, run with a stub
+``open3d`` module injected, returned on the same scenarios (tests/test_oracle_object_map.py, tests/golden/).  ``open3d`` itself (``open3d``,
 unpinned, README.md:45 / docker/Dockerfile) is ABSENT: ``dbscan_labels`` restates the published DBSCAN algorithm with
 Open3D's sequential cluster numbering (``PointCloud::ClusterDBSCAN``: radius neighbourhoods incl. the point itself, a point
 is core when it has >= min_points neighbours, clusters are grown one after the other from the lowest-index unlabelled core

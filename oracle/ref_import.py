@@ -1,7 +1,8 @@
-"""Import the REAL reference classes from /root/reference (build container only).
+"""Import the REAL reference classes from a checkout of the original vlfm repository.
 
-TEST INFRASTRUCTURE.  /root/reference does not exist on the GPU box: nothing that runs
-there may call this module (tests that use it are skipped when the tree is absent).
+TEST INFRASTRUCTURE, used only by oracle/make_golden.py to write tests/golden/: the tests
+compare against those stored outputs and never import the reference.  The checkout is
+named by the VLFM_REFERENCE environment variable.
 
 ``vlfm.mapping.value_map`` imports cleanly (cv2 + numpy only).
 ``vlfm.mapping.obstacle_map`` needs ``frontier_exploration`` (third-party, unpinned
@@ -15,7 +16,7 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = "/root/reference"
+REFERENCE_ROOT = os.environ.get("VLFM_REFERENCE", "")
 
 
 def available() -> bool:
@@ -55,6 +56,25 @@ def obstacle_map_class():
     from vlfm.mapping.obstacle_map import ObstacleMap  # type: ignore
 
     return ObstacleMap
+
+
+def base_map_class():
+    _ensure_path()
+    from vlfm.mapping.base_map import BaseMap  # type: ignore
+
+    return BaseMap
+
+
+def frontier_map_class(encoder_cls):
+    """vlfm.mapping.frontier_map with its HTTP BLIP-2 client replaced by ``encoder_cls`` (a stub ``vlfm.vlm.blip2itm``)."""
+    _ensure_path()
+    stub = types.ModuleType("vlfm.vlm.blip2itm")
+    stub.BLIP2ITMClient = encoder_cls
+    sys.modules["vlfm.vlm.blip2itm"] = stub
+    sys.modules.pop("vlfm.mapping.frontier_map", None)
+    from vlfm.mapping.frontier_map import FrontierMap  # type: ignore
+
+    return FrontierMap
 
 
 def geometry_utils():

@@ -15,7 +15,3 @@ def pytest_configure(config):
 @pytest.fixture(scope="session")
 def golden_dir():
     return os.path.join(ROOT, "tests", "golden")
-
-
-def has_reference() -> bool:
-    return os.path.isdir("/root/reference/vlfm/mapping")

@@ -1,10 +1,11 @@
-"""BaseMap conversions (vlfm/mapping/base_map.py:35-60): explicit formulae everywhere, the live reference class where present."""
-import sys
+"""BaseMap conversions (vlfm/mapping/base_map.py:35-60): explicit formulae, and what the reference class returned for the same
+points (stored under tests/golden/)."""
+import os
 
 import numpy as np
 import pytest
 
-from conftest import has_reference
+from oracle import golden
 from vlfm_b200.mapping.base_map import BaseMap
 
 
@@ -40,16 +41,15 @@ def test_conversions_match_reference_arithmetic(size, ppm):
     assert m._camera_positions == []
 
 
-@pytest.mark.skipif(not has_reference(), reason="/root/reference not present")
-def test_conversions_match_live_reference_class():
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    from vlfm.mapping.base_map import BaseMap as RefBaseMap  # type: ignore
-
+def run_conversions(m):
+    """`m` is a BaseMap-shaped object of size 1000."""
     rng = np.random.default_rng(5)
-    ref, got = RefBaseMap(size=1000), BaseMap(size=1000)
     pts = rng.uniform(-20, 20, (1000, 2))
-    assert np.array_equal(got._xy_to_px(pts), ref._xy_to_px(pts))
     cells = rng.uniform(0, 1000, (300, 2))
-    assert np.array_equal(got._px_to_xy(cells), ref._px_to_xy(cells))
-    assert np.array_equal(got._episode_pixel_origin, ref._episode_pixel_origin) and got.pixels_per_meter == ref.pixels_per_meter
+    return {"xy_to_px": m._xy_to_px(pts), "px_to_xy": m._px_to_xy(cells), "origin": np.asarray(m._episode_pixel_origin),
+            "ppm": np.array(m.pixels_per_meter)}
+
+
+def test_conversions_match_live_reference_class(golden_dir):
+    """The reference class's results on the same points are stored in tests/golden/ref_base_map.npz (oracle/make_golden.py)."""
+    golden.check(run_conversions(BaseMap(size=1000)), os.path.join(golden_dir, "ref_base_map.npz"))

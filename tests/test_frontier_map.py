@@ -1,13 +1,12 @@
 """FrontierMap (vlfm/mapping/frontier_map.py:10-77): host bookkeeping around one cosine call per update that introduces a
-new frontier.  Checked against explicit expectations everywhere, and against the REAL reference class (its HTTP encoder
-replaced by the same scripted one) where /root/reference exists."""
-import sys
-import types
+new frontier.  Checked against explicit expectations, and against what the REAL reference class (its HTTP encoder replaced by
+the same scripted one) returned for the same update streams, stored under tests/golden/."""
+import os
 
 import numpy as np
 import pytest
 
-from conftest import has_reference
+from oracle import golden
 from vlfm_b200.mapping.frontier_map import FrontierMap
 
 
@@ -51,34 +50,25 @@ def test_update_sort_reset_semantics():
     assert enc.calls == 2 and fm.frontiers == []
 
 
-@pytest.mark.skipif(not has_reference(), reason="/root/reference not present")
-@pytest.mark.parametrize("seed", [0, 1, 2])
-def test_matches_live_reference(seed):
-    stub = types.ModuleType("vlfm.vlm.blip2itm")
-    stub.BLIP2ITMClient = ScriptedEncoder
-    saved = {k: sys.modules.get(k) for k in ("vlfm.vlm.blip2itm", "vlfm.mapping.frontier_map")}
-    sys.modules["vlfm.vlm.blip2itm"] = stub
-    sys.modules.pop("vlfm.mapping.frontier_map", None)
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    try:
-        from vlfm.mapping.frontier_map import FrontierMap as RefFrontierMap  # type: ignore
+def run_stream(fm, seed):
+    """Frontier lists (in stored order) and sorted waypoints of `fm` (its encoder a ScriptedEncoder) after each update of the
+    seeded stream, concatenated over the updates."""
+    counts, xyz, cos, sorted_xyz, sorted_cos = [], [], [], [], []
+    for locs, img in _stream(seed):
+        fm.update(locs, img, "a chair")
+        counts.append(len(fm.frontiers))
+        xyz += [f.xyz for f in fm.frontiers]
+        cos += [f.cosine for f in fm.frontiers]
+        if fm.frontiers:
+            pts, vals = fm.sort_waypoints()
+            sorted_xyz.append(pts)
+            sorted_cos += vals
+    return {"counts": np.array(counts), "xyz": np.array(xyz).reshape(-1, 2), "cosine": np.array(cos, dtype=np.float64),
+            "sorted_xyz": np.concatenate(sorted_xyz).reshape(-1, 2), "sorted_cosine": np.array(sorted_cos, dtype=np.float64),
+            "encoder_calls": np.array(fm.encoder.calls)}
 
-        ref, got = RefFrontierMap(), FrontierMap(encoder=ScriptedEncoder())
-        ref.frontiers = []
-        for locs, img in _stream(seed):
-            ref.update(locs, img, "a chair")
-            got.update(locs, img, "a chair")
-            assert len(ref.frontiers) == len(got.frontiers)
-            for r, g in zip(ref.frontiers, got.frontiers):
-                assert np.array_equal(r.xyz, g.xyz) and r.cosine == g.cosine
-            if ref.frontiers:
-                (rp, rv), (gp, gv) = ref.sort_waypoints(), got.sort_waypoints()
-                assert rv == gv and np.array_equal(rp, gp)
-        assert ref.encoder.calls == got.encoder.calls
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
+
+@pytest.mark.parametrize("seed", [0, 1, 2])
+def test_matches_live_reference(golden_dir, seed):
+    """The reference class's lists on the same stream are stored in tests/golden/ref_frontier_map.npz (oracle/make_golden.py)."""
+    golden.check(run_stream(FrontierMap(encoder=ScriptedEncoder()), seed), os.path.join(golden_dir, "ref_frontier_map.npz"), f"s{seed}_")

@@ -1,10 +1,12 @@
 """Explore half of the obstacle map: the cv2-based restatement and the cv2-free one agree, and the reference's
-own ObstacleMap code (run with the restated frontier_exploration functions injected) agrees with both."""
+own ObstacleMap code (run with the restated frontier_exploration functions injected) agrees with both: its outputs are stored
+under tests/golden/."""
+import os
+
 import numpy as np
-import pytest
 
 import oracle.explore_oracle as ex
-from conftest import has_reference
+from oracle import golden
 from oracle.obstacle_map_oracle import ObstacleMapOracle
 from vlfm_b200.utils.synthetic import focal_from_hfov, trajectory
 
@@ -43,17 +45,21 @@ def test_backends_agree_at_the_map_border():
             assert np.array_equal(ea, eb) and fa.shape == fb.shape and np.array_equal(fa, fb) and np.array_equal(xa, xb)
 
 
-@pytest.mark.skipif(not has_reference(), reason="/root/reference not present")
-def test_reference_class_with_injected_functions():
-    from oracle import ref_import
-
-    RO = ref_import.obstacle_map_class()
-    r = RO(0.61, 0.88, 0.18, area_thresh=1.5, hole_area_thresh=-1, size=400)
-    o = ObstacleMapOracle(0.61, 0.88, 0.18, area_thresh=1.5, hole_area_thresh=-1, size=400)
+def run_reference_class_case(cls):
+    """explored area and frontiers of `cls` (an ObstacleMap-shaped class) after each of six seeded updates."""
+    m = cls(0.61, 0.88, 0.18, area_thresh=1.5, hole_area_thresh=-1, size=400)
     fx = focal_from_hfov(160)
-    for f in trajectory(7, 6, h=120, w=160, bound_m=4):
-        r.update_map(f.depth, f.tf, 0.5, 5.0, fx, fx, np.deg2rad(79))
-        o.update_map(f.depth, f.tf, 0.5, 5.0, fx, fx, np.deg2rad(79))
-        assert np.array_equal(r.explored_area, o.explored_area)
-        assert np.array_equal(np.asarray(r._frontiers_px), np.asarray(o._frontiers_px))
-        assert np.array_equal(np.asarray(r.frontiers), np.asarray(o.frontiers))
+    frames = trajectory(7, 6, h=120, w=160, bound_m=4)
+    out = {"inputs": np.array(golden.digest(*[a for f in frames for a in (f.depth, f.tf)]))}
+    for i, f in enumerate(frames):
+        m.update_map(f.depth, f.tf, 0.5, 5.0, fx, fx, np.deg2rad(79))
+        out[f"explored_{i}"] = m.explored_area.copy()
+        out[f"frontiers_px_{i}"] = np.asarray(m._frontiers_px).copy()
+        out[f"frontiers_{i}"] = np.asarray(m.frontiers).copy()
+    return out
+
+
+def test_reference_class_with_injected_functions(golden_dir):
+    """The reference's own ObstacleMap (restated frontier_exploration functions injected) on the same inputs is stored in
+    tests/golden/ref_explore.npz (oracle/make_golden.py)."""
+    golden.check(run_reference_class_case(ObstacleMapOracle), os.path.join(golden_dir, "ref_explore.npz"))

@@ -1,10 +1,13 @@
-"""oracle/object_map_oracle.py: DBSCAN restatement vs scikit-learn's implementation; the whole class vs the REAL reference
-class (vlfm/mapping/object_point_cloud_map.py) imported with a stub open3d."""
+"""oracle/object_map_oracle.py: DBSCAN restatement vs scikit-learn's implementation; the whole class vs what the REAL reference
+class (vlfm/mapping/object_point_cloud_map.py, imported with a stub open3d) returned on the same scenarios, stored under
+tests/golden/."""
+import os
+
 import cv2
 import numpy as np
 import pytest
 
-from conftest import has_reference
+from oracle import golden
 from oracle import object_map_oracle as om
 from vlfm_b200.utils.synthetic import focal_from_hfov, make_object_mask, trajectory
 
@@ -55,24 +58,27 @@ def _scenario(seed, steps=6, h=240, w=320):
     return out
 
 
-@pytest.mark.skipif(not has_reference(), reason="/root/reference not present")
-@pytest.mark.parametrize("use_dbscan", [True, False])
-def test_oracle_class_matches_the_reference_class(use_dbscan):
-    from oracle import ref_import
-
-    R = ref_import.object_map_module().ObjectPointCloudMap
+def run_scenarios(make, use_dbscan):
+    """has_object / cloud / best object / target cloud of the map `make()` returns, after each update of three seeded scenarios."""
+    out = {}
     for seed in range(3):
-        r, o = R(erosion_size=2), om.ObjectPointCloudMapOracle(erosion_size=2)
-        r.reset()
-        r.use_dbscan = o.use_dbscan = use_dbscan
-        for depth, mask, tf, fx in _scenario(seed):
-            for m in (r, o):
-                np.random.seed(7 + seed)
-                m.update_map("chair", depth, mask, tf, 0.5, 5.0, fx, fx)
-                m.update_explored(tf, 5.0, np.deg2rad(79))
-            assert r.has_object("chair") == o.has_object("chair")
-            if r.has_object("chair"):
-                assert np.array_equal(r.clouds["chair"], o.clouds["chair"])
-                pos = tf[:2, 3] + 0.3
-                assert np.array_equal(r.get_best_object("chair", pos), o.get_best_object("chair", pos))
-                assert np.array_equal(r.get_target_cloud("chair"), o.get_target_cloud("chair"))
+        m = make()
+        m.use_dbscan = use_dbscan
+        for i, (depth, mask, tf, fx) in enumerate(_scenario(seed)):
+            np.random.seed(7 + seed)
+            m.update_map("chair", depth, mask, tf, 0.5, 5.0, fx, fx)
+            m.update_explored(tf, 5.0, np.deg2rad(79))
+            key = f"s{seed}_{i}_"
+            out[key + "has"] = np.array(m.has_object("chair"))
+            if m.has_object("chair"):
+                out[key + "cloud"] = m.clouds["chair"]
+                out[key + "best"] = m.get_best_object("chair", tf[:2, 3] + 0.3)
+                out[key + "target"] = m.get_target_cloud("chair")
+    return out
+
+
+@pytest.mark.parametrize("use_dbscan", [True, False])
+def test_oracle_class_matches_the_reference_class(golden_dir, use_dbscan):
+    """The reference class's results on the same scenarios are stored in tests/golden/ref_object_map.npz (oracle/make_golden.py)."""
+    got = run_scenarios(lambda: om.ObjectPointCloudMapOracle(erosion_size=2), use_dbscan)
+    golden.check(got, os.path.join(golden_dir, "ref_object_map.npz"), f"dbscan{int(use_dbscan)}_")

@@ -1,25 +1,33 @@
+import os
+
 import numpy as np
 import pytest
 
-from conftest import has_reference
+from oracle import golden
 from oracle.obstacle_map_oracle import ObstacleMapOracle
 from vlfm_b200.utils.synthetic import focal_from_hfov, trajectory
 
+OBSTACLE_CASES = [(0, (240, 320), 600, 20), (2, (240, 320), 1500, 50)]
 
-@pytest.mark.skipif(not has_reference(), reason="/root/reference not present")
-@pytest.mark.parametrize("hole", [-1, 100000])
-def test_obstacle_half_matches_live_reference(hole):
-    from oracle import ref_import
 
-    RO = ref_import.obstacle_map_class()
-    for seed, (h, w), size, ppm in [(0, (240, 320), 600, 20), (2, (240, 320), 1500, 50)]:
-        r = RO(0.61, 0.88, 0.18, area_thresh=1.5, hole_area_thresh=hole, size=size, pixels_per_meter=ppm)
-        o = ObstacleMapOracle(0.61, 0.88, 0.18, area_thresh=1.5, hole_area_thresh=hole, size=size, pixels_per_meter=ppm)
+def run_obstacle_half(cls, hole):
+    """The obstacle / navigable grids of `cls` (an ObstacleMap-shaped class) after four seeded updates per case."""
+    out = {}
+    for seed, (h, w), size, ppm in OBSTACLE_CASES:
+        m = cls(0.61, 0.88, 0.18, area_thresh=1.5, hole_area_thresh=hole, size=size, pixels_per_meter=ppm)
         fx = focal_from_hfov(w)
-        for f in trajectory(seed, 4, h=h, w=w, bound_m=5):
-            r.update_map(f.depth, f.tf, 0.5, 5.0, fx, fx, np.deg2rad(79), explore=False)
-            o.update_map(f.depth, f.tf, 0.5, 5.0, fx, fx, np.deg2rad(79), explore=False)
-        assert np.array_equal(r._map, o._map) and np.array_equal(r._navigable_map, o._navigable_map)
+        frames = trajectory(seed, 4, h=h, w=w, bound_m=5)
+        for f in frames:
+            m.update_map(f.depth, f.tf, 0.5, 5.0, fx, fx, np.deg2rad(79), explore=False)
+        out[f"s{seed}_inputs"] = np.array(golden.digest(*[a for f in frames for a in (f.depth, f.tf)]))
+        out[f"s{seed}_map"], out[f"s{seed}_navigable"] = m._map, m._navigable_map
+    return out
+
+
+@pytest.mark.parametrize("hole", [-1, 100000])
+def test_obstacle_half_matches_live_reference(golden_dir, hole):
+    """The reference class's grids on the same inputs are stored in tests/golden/ref_obstacle_half.npz (oracle/make_golden.py)."""
+    golden.check(run_obstacle_half(ObstacleMapOracle, hole), os.path.join(golden_dir, "ref_obstacle_half.npz"), f"hole{hole}_")
 
 
 def _depth_with_holes(seed, h=60, w=80):

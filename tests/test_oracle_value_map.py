@@ -1,6 +1,5 @@
-"""Pin oracle/value_map_oracle.py: (1) against the committed fixtures generated from the
-real reference, (2) against the live reference when /root/reference exists,
-(3) cv2 and numpy primitive back-ends agree bit for bit."""
+"""Pin oracle/value_map_oracle.py against the committed fixtures generated from the real
+reference (oracle/make_golden.py), with the cv2 and the numpy primitive back-ends."""
 import glob
 import hashlib
 import os
@@ -8,7 +7,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import has_reference
+from oracle import golden
 from oracle.value_map_oracle import ValueMapOracle
 from vlfm_b200.utils.synthetic import trajectory
 
@@ -56,38 +55,42 @@ def test_oracle_matches_golden(golden_dir, prims):
         assert np.array_equal(sw, z["sorted_wp"]) and np.allclose(np.asarray(sv, float), z["sorted_val"], rtol=0, atol=0)
 
 
-@pytest.mark.skipif(not has_reference(), reason="/root/reference not present")
-def test_oracle_matches_live_reference():
-    from oracle import ref_import
+LIVE_CASES = [(1, False, "default", 700, 21), (2, True, "default", 500, 22)]
 
-    RV = ref_import.value_map_class()
-    for ch, maxc, fus, size, seed in [(1, False, "default", 700, 21), (2, True, "default", 500, 22)]:
-        RV._confidence_masks.clear()
-        r = RV(ch, size=size, use_max_confidence=maxc, fusion_type=fus)
-        o = ValueMapOracle(ch, size=size, use_max_confidence=maxc, fusion_type=fus, prims="numpy")
+
+def run_live_cases(make):
+    """make(channels, size, use_max_confidence, fusion_type) -> a value map; the grids after five seeded updates per case."""
+    out = {}
+    for ch, maxc, fus, size, seed in LIVE_CASES:
+        m = make(ch, size, maxc, fus)
         rng = np.random.default_rng(seed)
-        for f in trajectory(seed, 5, bound_m=size / 40 - 6):
-            v = rng.random(ch)
-            r.update_map(v, f.depth, f.tf, 0.5, 5.0, FOV)
-            o.update_map(v, f.depth, f.tf, 0.5, 5.0, FOV)
-        assert np.array_equal(r._map, o._map) and np.array_equal(r._value_map, o._value_map)
+        frames = trajectory(seed, 5, bound_m=size / 40 - 6)
+        for f in frames:
+            m.update_map(rng.random(ch), f.depth, f.tf, 0.5, 5.0, FOV)
+        out[f"s{seed}_inputs"] = np.array(_digest(frames))
+        out[f"s{seed}_conf"], out[f"s{seed}_value"] = m._map, m._value_map
+    return out
 
 
-@pytest.mark.skipif(not has_reference(), reason="/root/reference not present")
-def test_oracle_ppm40_matches_patched_reference():
-    """configs[4]/[5] geometry: the reference needs `pixels_per_meter` patched and its cone cache cleared
-    (value_map.py:65, :339); the oracle takes ppm as a parameter."""
-    from oracle import ref_import
-
-    RV = ref_import.value_map_class()
-    RV._confidence_masks.clear()
-    r = RV(1, size=1000, use_max_confidence=False)
-    r.pixels_per_meter = 40
-    o = ValueMapOracle(1, size=1000, use_max_confidence=False, pixels_per_meter=40, prims="numpy")
+def run_ppm40(make):
+    """make(size) -> a value map at 40 pixels per metre (configs[4]/[5] geometry)."""
+    m = make(1000)
     rng = np.random.default_rng(9)
-    for f in trajectory(62, 2, h=128, w=128, bound_m=6.0):
-        v = rng.random(1)
-        r.update_map(v, f.depth, f.tf, 0.5, 5.0, FOV)
-        o.update_map(v, f.depth, f.tf, 0.5, 5.0, FOV)
-    RV._confidence_masks.clear()
-    assert np.array_equal(r._map, o._map) and np.array_equal(r._value_map, o._value_map)
+    frames = trajectory(62, 2, h=128, w=128, bound_m=6.0)
+    for f in frames:
+        m.update_map(rng.random(1), f.depth, f.tf, 0.5, 5.0, FOV)
+    return {"inputs": np.array(_digest(frames)), "conf": m._map, "value": m._value_map}
+
+
+def test_oracle_matches_live_reference(golden_dir):
+    """The reference class's grids on the same inputs are stored in tests/golden/ref_value_map_live.npz (oracle/make_golden.py)."""
+    got = run_live_cases(lambda ch, size, maxc, fus: ValueMapOracle(ch, size=size, use_max_confidence=maxc, fusion_type=fus,
+                                                                      prims="numpy"))
+    golden.check(got, os.path.join(golden_dir, "ref_value_map_live.npz"))
+
+
+def test_oracle_ppm40_matches_patched_reference(golden_dir):
+    """configs[4]/[5] geometry: the reference needs `pixels_per_meter` patched and its cone cache cleared
+    (value_map.py:65, :339); the oracle takes ppm as a parameter.  Reference grids: tests/golden/ref_value_map_ppm40.npz."""
+    got = run_ppm40(lambda size: ValueMapOracle(1, size=size, use_max_confidence=False, pixels_per_meter=40, prims="numpy"))
+    golden.check(got, os.path.join(golden_dir, "ref_value_map_ppm40.npz"))
